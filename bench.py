@@ -2,7 +2,7 @@
 """Headline benchmark: frames/s of one BLSTM-CTC training step (BASELINE.json config 2:
 5x512 BLSTM, 80-d input, T=1000, B=64 per GPU, 28 chars + blank), data-parallel over N GPUs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = forward (5 BLSTM layers + output FC) + CTC loss/grad + backward (BPTT + weight
 gradients) + per-tensor clip_by_norm + gradient all-reduce (N>1) + RMSProp update.
@@ -141,6 +141,45 @@ def cpu_arm_record(v, dt, threads, nsteps):
                     "TensorFlow itself is not installable here" % threads}
 
 
+DUMP_SAMPLE = 1 << 20      # elements of the flat parameter / gradient buffers written by --dump-outputs
+
+
+def restore_initial_state(model, params0):
+    """Parameters as constructed and optimizer slots as created, so that the step that follows starts from the
+    same state in every run.  Without it the last step's inputs would be the product of every earlier step, and
+    those carry the run-to-run rounding of the atomic gradient reductions (measured on a B200 at 1000 W: 1e-4
+    relative in the loss after a dozen steps, near 10 % after fifty)."""
+    from tensorflow_end2end_speech_recognition_b200.models.model_base import OPTIMIZER_CLS_NAMES
+    model.flat_params.copy_(params0)
+    model._params_version += 1
+    opt = model.optimizer
+    if opt.state0 is not None:
+        opt.state0.fill_(OPTIMIZER_CLS_NAMES[opt.name][2])
+    if opt.state1 is not None:
+        opt.state1.zero_()
+    opt.global_step = 0
+
+
+def dump_outputs(out_dir, model, loss, logits):
+    """What a caller of the timed step receives after its last step: the mean CTC loss, the per-utterance
+    losses, the logits [T,B,C], and the parameters the optimizer updated (with the clipped gradients it
+    applied).  The flat buffers (over 100 MB each) are sampled at fixed indices (seed 0, sorted), so that two
+    builds write arrays that compare element for element.  About 16 MB in all."""
+    import torch
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    n = model.flat_params.numel()
+    idx = np.sort(np.random.RandomState(0).choice(n, min(n, DUMP_SAMPLE), replace=False))
+    idx_dev = torch.from_numpy(idx).to(model.flat_params.device)
+    arrays = {"loss": loss.detach().reshape(1).double(),
+              "ctc_losses": model.ctc_losses.detach().float(),
+              "logits": logits.detach().float(),
+              "params_sample": model.flat_params[idx_dev].float(),
+              "grads_sample": model.flat_grads[idx_dev].float()}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def run_reference(args):
     """--impl reference: CPU port of the reference step, rank 0 only.  One step = the bounded sample
     CPU_B x CPU_T (T stays 1000); at ~1 minute per step the arm times min(K, 2) steps after min(W, 1)
@@ -177,7 +216,14 @@ def main():
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--precision", default="bf16")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0): loss, ctc_losses, "
+                         "logits, and a fixed seeded sample of the updated parameters and of the gradients; that "
+                         "step starts from the seeded initial parameters and optimizer state, restored inside the "
+                         "timed region (one parameter-buffer copy and one optimizer-slot fill)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -217,6 +263,8 @@ def main():
             except Exception as e:          # keep the run alive on the torch path, and say so
                 comm, comm_kind = None, "torch.distributed all_reduce (C-ABI communicator failed: %s)" % (e,)
     model.set_data_parallel(world, comm=comm)
+    # the seeded initial parameters, restored before the last timed step of a --dump-outputs run
+    params0 = model.flat_params.clone() if args.dump_outputs else None
     # weak scaling: every rank gets its own 64-utterance shard (np.array_split of a 64*N batch,
     # utils/dataset/ctc.py:171-177); strong scaling: its slice of the one 64-utterance batch
     x, seq, labels = make_batch(1234 + rank, B, T, D, CFG["num_classes"], CFG["label_min"], CFG["label_max"])
@@ -224,9 +272,12 @@ def main():
     seq_host = torch.from_numpy(seq).pin_memory()
     x_dev, seq_dev = x_host.to(dev), seq_host.to(dev)
 
+    last = {}
+
     def step(xin, sin):
-        loss, _ = model.compute_loss(xin, labels, sin, keep_prob=CFG["keep_prob"])
+        loss, logits = model.compute_loss(xin, labels, sin, keep_prob=CFG["keep_prob"])
         model.train(loss, CFG["optimizer"], CFG["lr"])
+        last["outputs"] = (loss, logits)
         return loss
 
     def barrier():
@@ -247,7 +298,6 @@ def main():
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
-    last = {}
     # e2e: every step copies ITS batch host -> device (pinned, on the prefetcher's side stream, issued one step
     # ahead so that it overlaps the previous step) and reads ITS loss device -> host (asynchronous copy into
     # pinned memory, consumed one step later so the host never drains the launch queue); both transfers of
@@ -291,15 +341,23 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    l0 = lib.b2_launch_count()
-    ms_dev = timed(lambda: step(x_dev, seq_dev), args.steps)
-    launches = (lib.b2_launch_count() - l0) // max(args.steps, 1)
+    try:
+        l0 = lib.b2_launch_count()
+        ms_dev = timed(lambda: step(x_dev, seq_dev), args.steps)
+        launches = (lib.b2_launch_count() - l0) // args.steps
 
-    def e2e_loop_body():
-        e2e_step()
-    ms_e2e = timed(e2e_loop_body, args.steps)
-    e2e_flush()
-    clocks = sampler.stop() if rank == 0 else None
+        last_i = state["i"] + args.steps - 1
+
+        def e2e_loop_body():
+            if params0 is not None and state["i"] == last_i:
+                restore_initial_state(model, params0)
+            e2e_step()
+        ms_e2e = timed(e2e_loop_body, args.steps)
+        e2e_flush()
+    finally:
+        clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, *last["outputs"])
 
     frames = (CFG["B"] if SCALING == "strong" else B * world) * T
     value = frames * args.steps / (ms_dev / 1e3)

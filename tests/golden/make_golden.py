@@ -4,8 +4,8 @@ decoders (the only part of the hot path that imports without TensorFlow):
     models/ctc/decoders/greedy_decoder.py:19-50      GreedyDecoder.__call__
     models/ctc/decoders/beam_search_decoder.py:53-152 BeamSearchDecoder.__call__
 
-Run in the build container (needs /root/reference on sys.path):
-    python tests/golden/make_golden.py
+Run with a checkout of the reference repository:
+    python tests/golden/make_golden.py <reference checkout>
 The reference is called one utterance at a time, its canonical usage
 (examples/librispeech/metrics/ctc.py:214-218).
 """
@@ -15,7 +15,7 @@ import warnings
 
 import numpy as np
 
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, sys.argv[1])
 warnings.filterwarnings("ignore")
 from models.ctc.decoders.beam_search_decoder import BeamSearchDecoder  # noqa: E402
 from models.ctc.decoders.greedy_decoder import GreedyDecoder  # noqa: E402

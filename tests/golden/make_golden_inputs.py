@@ -5,15 +5,15 @@ transforms (they import without TensorFlow):
     utils/io/inputs/splicing.py:9-73          do_splice
 
 and, on the way, asserts that the closed-form restatement in oracle/inputs.py reproduces them
-bit for bit on a wider random sweep.  Run in the build container:
-    python tests/golden/make_golden_inputs.py
+bit for bit on a wider random sweep.  Run with a checkout of the reference repository:
+    python tests/golden/make_golden_inputs.py <reference checkout>
 """
 import os
 import sys
 
 import numpy as np
 
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, sys.argv[1])
 from utils.io.inputs.frame_stacking import stack_frame  # noqa: E402
 from utils.io.inputs.splicing import do_splice  # noqa: E402
 
